@@ -2,7 +2,7 @@
 """bench.py -- frames/s of the ProPainter inference hot path on B200 (contract in the task statement).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c1|c3|c4|c5] [--no-cpu-baseline]
-                  [--no-gpu-reference] [--no-strong] [--shard]
+                  [--no-gpu-reference] [--no-strong] [--shard] [--dump-outputs DIR]
 
 A "step" is one full pass of stages 1-4 (RAFT flow -> flow completion -> image propagation ->
 sliding-window generator + compositing) over one synthetic clip.  N=1 workload = BASELINE.json
@@ -17,6 +17,10 @@ propainter_b200/dist.py (point-to-point halo exchange over NCCL), at every N inc
 of the long-clip configuration can be read off the per-N lines.
 --impl reference: the oracle (CPU restatement of the reference's PyTorch path) on the host cores
 over a bounded sample of the same workload.
+--dump-outputs DIR: after the timed steps, rank 0 writes the composited video its last timed step returned (see
+dump_outputs); inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
+Two runs of one build (C2, one B200 at 1000 W) differed by one level in 0.2 % of the sampled values: compare with a
+tolerance of one level.
 """
 import argparse
 import json
@@ -44,6 +48,7 @@ WORKLOADS = {
 }
 STRONG_WORKLOAD = "c4"     # the long clip of BASELINE.json configs[3] that `strong` shards over the ranks
 CPU_SAMPLE_FRAMES = 6      # bounded sample of the same workload for the CPU arm (full clip ~ 10 min of CPU)
+DUMP_SAMPLE = 4 << 20      # --dump-outputs: elements kept of a larger output (4 B value + 8 B index each: 48 MiB)
 
 
 def peaks():
@@ -238,6 +243,20 @@ def cpu_baseline(wl):
             "sample": f"first {T} frames of the workload clip, full 4-stage pipeline once ({dt:.1f} s), {cores} host threads"}
 
 
+def dump_outputs(out_dir, comp):
+    """The composited uint8 video [T,H,W,3] as float32 <out_dir>/comp.npy.  A video of more than DUMP_SAMPLE elements is
+    written as a fixed sample: its values at DUMP_SAMPLE flat indices drawn once with seed 0, in ascending order, and those
+    indices as float64 comp_index.npy."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    if comp.numel() > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(comp.numel(), DUMP_SAMPLE, replace=False))
+        np.save(os.path.join(out_dir, "comp_index.npy"), idx.astype(np.float64))
+        comp = comp.reshape(-1)[torch.from_numpy(idx).to(comp.device)]
+    np.save(os.path.join(out_dir, "comp.npy"), comp.cpu().numpy().astype(np.float32))
+
+
 def _time_kernel(torch, fn, reps=10):
     """CUDA events on the launch stream (= torch's current stream, which ops.* launch on), L2 flushed between reps."""
     flush = torch.empty(64 * 1024 * 1024, device="cuda")
@@ -414,9 +433,16 @@ def run_ours(args, wl):
         from propainter_b200.dist import ShardedProPainter
         runner = ShardedProPainter(pipe)
 
+    last = {}                                                  # the latest resident step's result, for --dump-outputs
+
     def step_resident():
         r = runner(u8_dev, fm_dev, md_dev, cfg)
-        return r[0] if shard else r
+        last["comp"] = r[0] if shard else r
+        return last["comp"]
+
+    def dump_last():
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, last["comp"])
 
     def step_e2e():
         r = runner(u8_host, fm_host, md_host, cfg)             # H2D inside
@@ -472,7 +498,7 @@ def run_ours(args, wl):
                 if e2e:
                     outs[k].copy_(pipes[k](u8_host, fm_host, md_host, cfg), non_blocking=True)
                 else:
-                    pipes[k](u8_dev, fm_dev, md_dev, cfg)
+                    last["comp"] = pipes[k](u8_dev, fm_dev, md_dev, cfg)
             main = torch.cuda.current_stream()
             for st in streams:
                 st.wait_stream(main)
@@ -508,9 +534,11 @@ def run_ours(args, wl):
         ms_one, _, _ = timed(step_resident, min(args.steps, 3), args.warmup)          # latency of one clip alone, for the record
         single = {"ms_per_clip": ms_one / min(args.steps, 3), "frames_per_s": wl["T"] * min(args.steps, 3) / (ms_one * 1e-3)}
         ms_total, launches, clocks = timed_pipelined(False, args.steps, args.warmup)
+        dump_last()
         ms_e2e, _, _ = timed_pipelined(True, args.steps, 1)
     else:
         ms_total, launches, clocks = timed(step_resident, args.steps, args.warmup, True)
+        dump_last()
         ms_e2e, _, _ = timed(step_e2e, args.steps, 1)
     strong = None
     frames_total = wl["T"] * (1 if shard else world) * args.steps
@@ -590,7 +618,12 @@ def main():
     ap.add_argument("--clips-in-flight", type=int, default=1,
                     help="engine replicas per GPU working on consecutive clips concurrently (each step is still one full clip)")
     ap.add_argument("--shard", action="store_true", help="N>1: cooperate on ONE clip (strong scaling) instead of one clip per rank")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the composited video of the last timed step under DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl)

@@ -1,8 +1,7 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference modules (imported read-only from
-/root/reference) in the authoring container.  Not runnable on the GPU box (no /root/reference there);
-the committed fixtures are what travels.
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference modules, imported read-only from a checkout of
+sczhou/ProPainter.  The tests only read the committed fixtures; this script is how they were made.
 
-    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
+    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py --reference <ProPainter checkout> [--cases ...]
 
 Weights: the seeded synthetic state_dicts of the product's ParamNets (seeds 1/2/3), loaded into the
 reference modules with strict=True -- which also proves the state_dict schema is identical.
@@ -18,17 +17,16 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
-sys.path.insert(1, "/root/reference")
-
-from RAFT import RAFT as RefRAFT  # noqa: E402
-from model.propainter import InpaintGenerator as RefGen  # noqa: E402
-from model.recurrent_flow_completion import RecurrentFlowCompleteNet as RefRFC  # noqa: E402
 
 from propainter_b200 import schemas, synth  # noqa: E402
 from propainter_b200._params import ParamNet  # noqa: E402
 
 
-def build_reference():
+def build_reference(ref_dir):
+    sys.path.insert(1, ref_dir)
+    from RAFT import RAFT as RefRAFT
+    from model.propainter import InpaintGenerator as RefGen
+    from model.recurrent_flow_completion import RecurrentFlowCompleteNet as RefRFC
     sds = {"raft": ParamNet(schemas.raft_schema(), seed=1).state_dict(),
            "rfc": ParamNet(schemas.rfc_schema(), seed=2).state_dict(),
            "gen": ParamNet(schemas.generator_schema(), seed=3).state_dict()}
@@ -133,14 +131,17 @@ def reference_pipeline(nets, u8, flow_masks, masks_dilated, raft_iter=20, neighb
     return np.stack(comp, 0), dict(gt_f=gt[0], gt_b=gt[1], pred_f=pred[0], pred_b=pred[1], upd_f=upd_f, upd_m=upd_m, win0=first_window)
 
 
-def summarize(name, comp, st, out_dir, stride=4, md=None):
-    """stride: spatial subsampling of the stage tensors.  With `md` (the dilated masks) only the pixels of the composited
-    video inside the holes are stored (`comp_holes`, in np.nonzero order): outside them the video equals the input clip,
-    which the test regenerates from the seed -- this keeps the 80-frame fixtures at a few MB."""
-    sub = lambda z: z[..., ::stride, ::stride].contiguous().numpy()
+def summarize(name, comp, st, out_dir, u8, md=None, stride=4, frame_step=1, hole_step=1):
+    """stride / frame_step: spatial / temporal subsampling of the stage tensors.  With `md` (the dilated masks) only the
+    pixels of the composited video inside the holes are stored, every `hole_step`-th of them in np.nonzero order
+    (`comp_holes`): outside them the video equals the input clip, which the test regenerates from the seed.  The steps
+    keep every fixture under 1 MB."""
+    sub = lambda z: z[:, ::frame_step, :, ::stride, ::stride].contiguous().numpy()
     if md is not None:
         sel = md[0, :, 0].numpy() > 0
-        extra = dict(comp_holes=comp[sel], stride=np.array(stride))
+        assert np.array_equal(comp[~sel], u8[~sel])
+        extra = dict(comp_holes=comp[sel][::hole_step], stride=np.array(stride), frame_step=np.array(frame_step),
+                     hole_step=np.array(hole_step))
     else:
         extra = dict(comp=comp)
     np.savez_compressed(
@@ -154,26 +155,30 @@ CASES = {
     # BASELINE.json configs[0]: 8-frame 128x128 clip + square mask (reduced RAFT iterations keep it CPU-cheap)
     "c1_8x128x128_square_it6": dict(T=8, H=128, W=128, mask="square", raft_iter=6, sub=80),
     # T > subvideo_length: halo chunking of stages 2/3 and bounded ref selection
-    "chunk_23x128x128_ellipse_it2_sub10": dict(T=23, H=128, W=128, mask="ellipse", raft_iter=2, sub=10),
+    "chunk_23x128x128_ellipse_it2_sub10": dict(T=23, H=128, W=128, mask="ellipse", raft_iter=2, sub=10, holes=True),
     # BASELINE.json configs[1] = the benchmarked workload, full size (~10 min of CPU each; `--cases` selects)
-    "c2_80x240x432_ellipse_it20": dict(T=80, H=240, W=432, mask="ellipse", raft_iter=20, sub=80, stride=8, holes=True),
+    "c2_80x240x432_ellipse_it20": dict(T=80, H=240, W=432, mask="ellipse", raft_iter=20, sub=80, stride=16, frame_step=2,
+                                       holes=True, hole_step=8),
     # configs[2] clip: 25 % border mask (video completion); the reference's CPU path is fp32 (inference_propainter.py:221-222)
-    "c3_80x240x432_border_it20": dict(T=80, H=240, W=432, mask="border", raft_iter=20, sub=80, stride=8, holes=True),
+    "c3_80x240x432_border_it20": dict(T=80, H=240, W=432, mask="border", raft_iter=20, sub=80, stride=16, frame_step=2,
+                                      holes=True, hole_step=24),
 }
 DEFAULT_CASES = ["c1_8x128x128_square_it6", "chunk_23x128x128_ellipse_it2_sub10"]
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
+    ap.add_argument("--reference", required=True, help="checkout of sczhou/ProPainter whose modules produce the fixtures")
     ap.add_argument("--cases", nargs="*", default=DEFAULT_CASES, choices=list(CASES))
     ap.add_argument("--threads", type=int, default=0)
     a = ap.parse_args()
     if a.threads:
         torch.set_num_threads(a.threads)
-    nets = build_reference()
+    nets = build_reference(a.reference)
     out_dir = os.path.dirname(os.path.abspath(__file__))
     for name in a.cases:
         c = CASES[name]
         u8, fm, md = synth.make_clip(c["T"], c["H"], c["W"], mask=c["mask"], seed=0)
         comp, st = reference_pipeline(nets, u8, fm, md, raft_iter=c["raft_iter"], subvideo_length=c["sub"])
-        summarize(name, comp, st, out_dir, stride=c.get("stride", 4), md=md if c.get("holes") else None)
+        summarize(name, comp, st, out_dir, u8, md=md if c.get("holes") else None, stride=c.get("stride", 4),
+                  frame_step=c.get("frame_step", 1), hole_step=c.get("hole_step", 1))
         print(name, "done", comp.shape, os.path.getsize(os.path.join(out_dir, name + ".npz")) // 1024, "KiB")

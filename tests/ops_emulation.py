@@ -271,3 +271,7 @@ def install(monkeypatch, hostsim):
     for name, fn in list(locals().items()):
         if callable(fn) and hasattr(ops, name) and not name.startswith("_"):
             monkeypatch.setattr(ops, name, fn)
+    # plan choices are keyed by shape, not device: ones measured by GPU tests earlier in the session would replay
+    # CUDA-only library plans (cuDNN's fused conv-bias-ReLU) on these CPU tensors
+    from propainter_b200 import autotune
+    monkeypatch.setattr(autotune, "_choice", {})

@@ -26,7 +26,12 @@ def load_case(name):
     c = CASES[name]
     g = np.load(os.path.join(GOLD, name + ".npz"))
     u8, fm, md = synth.make_clip(c["T"], c["H"], c["W"], mask=c["mask"], seed=0)
-    return c, g, u8, fm, md
+    if "comp" in g.files:
+        ref = g["comp"]
+    else:                                                  # stored inside the holes only: outside them it is the input clip
+        ref = u8.copy()
+        ref[md[0, :, 0].numpy() > 0] = g["comp_holes"]
+    return c, g, ref, u8, fm, md
 
 
 def compare_stages(g, st, tol):
@@ -44,15 +49,15 @@ def compare_stages(g, st, tol):
 
 @pytest.mark.parametrize("name", list(CASES))
 def test_oracle_reproduces_reference_golden(name):
-    c, g, u8, fm, md = load_case(name)
+    c, g, ref, u8, fm, md = load_case(name)
     comp, st = pipeline_ref.run_pipeline(seeded_state_dicts(), u8, fm, md, raft_iter=c["raft_iter"], subvideo_length=c["sub"],
                                          return_stages=True)
     res = compare_stages(g, st, {"gt": 1e-5, "pred": 1e-5})
     assert res["upd_m_mismatch"] == 0.0
     # the generator differs from the reference by ~1e-6 (summation order); the uint8 truncation of
     # inference_propainter.py:443 may then flip an isolated pixel by one level
-    d = np.abs(comp.astype(int) - g["comp"].astype(int))
-    assert d.max() <= 1 and (d > 0).mean() < 1e-4 and ops_ref.psnr_u8(comp, g["comp"]) > 85.0
+    d = np.abs(comp.astype(int) - ref.astype(int))
+    assert d.max() <= 1 and (d > 0).mean() < 1e-4 and ops_ref.psnr_u8(comp, ref) > 85.0
 
 
 def test_psnr_definition():
